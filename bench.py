@@ -394,7 +394,17 @@ class Case:
         out["tolerance"] = PARITY_TOL
         return out
 
-    def measure(self, steps, warmup, sampler=None):
+    def outputs(self):
+        """what the last GN step through the C ABI left for its caller: the committed system (dmv_ba_accumulate), the per-residual and
+        per-point results and the updated depths; integer outputs as float64"""
+        ba = self.ba
+        out = ba.accumulate()
+        out.update(ba.residual_outputs())
+        out.update({"pt_" + k: v for k, v in ba.point_outputs().items()})
+        out["idepth"], out["idepth_zero"] = ba.get_idepth()
+        return {k: np.asarray(v, np.float64 if np.asarray(v).dtype.kind in "iub" else None) for k, v in out.items()}
+
+    def measure(self, steps, warmup, sampler=None, dump=None):
         ba, D, x = self.ba, self.D, self.x
         for _ in range(max(3, warmup)):
             ba.gn_step(x, self.k8, self.precalc, self.TH)
@@ -421,6 +431,8 @@ class Case:
         D.barrier()
         if sampler:
             sampler.mark(tw0, time.perf_counter())
+        if dump is not None:
+            dump.update(self.outputs())
         e2e_ms = D.max(e2e_ms_c)
         launches = int(ba.launch_count() - launches0)
         ba.set_timing(True)
@@ -538,6 +550,24 @@ def coarse_record(local_rank, peak):
     return out
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, arrays):
+    """writes each array as d/<name>.npy (float32 / float64).  Above DUMP_BYTES in all, every array is cut to the same fixed, seeded
+    sample of rows (its first axis), and the sampled row indices are written beside it as <name>_rows.npy (float64 indices take at most
+    twice the bytes of the rows they index, hence a third of the budget for the rows themselves)."""
+    os.makedirs(d, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in sorted(arrays.items()):
+        if total > DUMP_BYTES and a.ndim > 0 and a.shape[0] > 1:
+            k = max(1, int(a.shape[0] * DUMP_BYTES / (3 * total)))
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], k, replace=False))
+            a = a[rows]
+            np.save(os.path.join(d, f"{name}_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(d, f"{name}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -552,6 +582,8 @@ def main():
     ap.add_argument("--batch", type=int, default=8, help="windows per launch of the batched roofline record (N = 1 only); 0 = skip")
     ap.add_argument("--no-extras", action="store_true", help="skip the strong-scaling / config-4 / batched side records")
     ap.add_argument("--ref-courtesy", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline window returned to its caller as DIR/<name>.npy (rank 0)")
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "nccl"],
                     help="N>1: all-reduce of the system inside the kernel over NVLink peer memory (CUDA IPC) or by NCCL behind it")
     args = ap.parse_args()
@@ -579,7 +611,10 @@ def main():
     # ---------------- headline: weak scaling, NPTS points per rank
     C = Case(D, rank, world, local_rank, NPTS * world, args.chunk, args.exchange)
     parity = C.parity()
-    m = C.measure(args.steps, args.warmup, sampler)
+    dump = {} if args.dump_outputs and rank == 0 else None
+    m = C.measure(args.steps, args.warmup, sampler, dump)
+    if dump is not None:
+        dump_outputs(args.dump_outputs, dump)
     balg = algorithmic_bytes(C.nres_local, len(C.Wr["host"]), NF)
     exchange, r0, nres_total, nres_local = C.exchange, C.r0, C.nres_total, C.nres_local
     Wfull = C.Wfull

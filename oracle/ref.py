@@ -140,6 +140,7 @@ def make_images(img, K):
     for l in range(lv):
         sz = (w >> l) * (h >> l) * 3
         res.append(out[off:off + sz].reshape(h >> l, w >> l, 3))
+        res[-1][[0, -1], :, 1:] = 0   # gradients of the first and last row: left uninitialised by FrameHessian::makeImages (HessianBlocks.cpp:L169-179)
         off += sz
     return res
 

@@ -85,7 +85,7 @@ def _worker(rank, world, port, cfg, mode, q):
 def test_sharded_exchange(orc, synth, world, mode):
     import dmvio_b200.capi as capi
     if capi.lib().dmv_device_count() < world:
-        pytest.skip(f"needs {world} GPUs (run with gpurun --gpus {world})")
+        pytest.skip(f"needs {world} GPUs")
     import torch.multiprocessing as mp
     cfg = dict(nf=5, npts=901, seed=17) if world == 2 else dict(nf=7, npts=250 * world + 3, seed=17 + world)
     ctx = mp.get_context("spawn")
@@ -185,7 +185,7 @@ def test_window_ba_sharded(synth, world, mode):
     import dmvio_b200.capi as capi
     import dmvio_b200.hostapi as hostapi
     if capi.lib().dmv_device_count() < world:
-        pytest.skip(f"needs {world} GPUs (run with gpurun --gpus {world})")
+        pytest.skip(f"needs {world} GPUs")
     import torch.multiprocessing as mp
     cfg = dict(nf=6, npts=500 + world, seed=31, state_noise=1e-3, hosts="all")
     ctx = mp.get_context("spawn")
