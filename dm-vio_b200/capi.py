@@ -110,6 +110,17 @@ class CTConfig(C.Structure):
     _fields_ = [("w", C.c_int), ("h", C.c_int), ("levels", C.c_int), ("max_points", C.c_int), ("device", C.c_int)]
 
 
+class CTTrackArgs(C.Structure):
+    _fields_ = [("R", C.c_double * 9), ("t", C.c_double * 3), ("a", C.c_double), ("b", C.c_double), ("ref_a", C.c_double), ("ref_b", C.c_double),
+                ("ref_exposure", C.c_float), ("new_exposure", C.c_float), ("coarseCutoffTH", C.c_float), ("affineOptModeA", C.c_float),
+                ("affineOptModeB", C.c_float), ("coarsestLvl", C.c_int), ("minResForAbort", C.c_double * 5)]
+
+
+class CTTrackResult(C.Structure):
+    _fields_ = [("R", C.c_double * 9), ("t", C.c_double * 3), ("a", C.c_double), ("b", C.c_double), ("lastResiduals", C.c_double * 5),
+                ("flowIndicators", C.c_double * 3), ("trackingGood", C.c_int), ("iterations", C.c_int), ("evaluations", C.c_int), ("status", C.c_int)]
+
+
 class CIEvalArgs(C.Structure):
     _fields_ = [("level", C.c_int), ("RKi", C.c_float * 9), ("t_d", C.c_double * 3), ("t_log", C.c_double * 3), ("r2new_aff", C.c_float * 2),
                 ("huberTH", C.c_float), ("alphaK", C.c_float), ("alphaW", C.c_float), ("couplingWeight", C.c_float),
@@ -201,6 +212,7 @@ def lib():
         L.dmv_ct_upload_new_image.argtypes = [vp, f32p]
         L.dmv_ct_set_huber.argtypes = [vp, C.c_float]
         L.dmv_ct_calc_res_gs.argtypes = [vp, C.c_int, f32p, f32p, f32p, C.c_float, C.c_float, C.c_int, f64p, f64p, f64p, C.POINTER(C.c_int)]
+        L.dmv_ct_track.argtypes = [vp, C.POINTER(CTTrackArgs), C.POINTER(CTTrackResult)]
         L.dmv_ct_init_points.argtypes = [vp, C.c_int, i32p, i32p, f32p, f32p, f32p, f32p, i32p]
         L.dmv_ct_trace_points.argtypes = [vp, C.POINTER(IPPoints), f32p, f32p, f32p, vp]
         L.dmv_ct_trace_points_multi.argtypes = [vp, C.c_int, vp, f32p, vp]
@@ -497,6 +509,22 @@ class CT:
         check(self.L.dmv_ct_calc_res_gs(self.h, lvl, _c(RKi, np.float32).reshape(-1), _c(t, np.float32), _c(affLL, np.float32), b0, cutoff,
                                         int(want_gs), res6, H, b, C.byref(n)))
         return res6, H.reshape(8, 8), b, n.value
+
+    def track(self, R, t, a, b, coarsest=None, minRes=None, ref_a=0.0, ref_b=0.0, ref_exposure=1.0, new_exposure=1.0, cutoff=20.0,
+              affModeA=1e12, affModeB=1e8):
+        """trackNewestCoarse in one launch (dmv_ct_track) from refToNew (R, t) and aff_g2l (a, b); minRes = minResForAbort (NaN = never abort).
+        Returns the dmv_ct_track_result fields as a dict."""
+        args = CTTrackArgs()
+        args.R[:] = [float(x) for x in np.asarray(R, np.float64).reshape(-1)]
+        args.t[:] = [float(x) for x in np.asarray(t, np.float64).reshape(-1)]
+        args.a, args.b, args.ref_a, args.ref_b = a, b, ref_a, ref_b
+        args.ref_exposure, args.new_exposure, args.coarseCutoffTH, args.affineOptModeA, args.affineOptModeB = ref_exposure, new_exposure, cutoff, affModeA, affModeB
+        args.coarsestLvl = self.levels - 1 if coarsest is None else coarsest
+        args.minResForAbort[:] = [float(x) for x in (np.full(5, np.nan) if minRes is None else np.asarray(minRes, np.float64))]
+        r = CTTrackResult()
+        check(self.L.dmv_ct_track(self.h, C.byref(args), C.byref(r)))
+        return dict(R=np.array(r.R).reshape(3, 3), t=np.array(r.t), a=r.a, b=r.b, lastResiduals=np.array(r.lastResiduals), flow=np.array(r.flowIndicators),
+                    good=r.trackingGood, iterations=r.iterations, evaluations=r.evaluations, status=r.status)
 
     def make_coarse_depth(self, Ku, Kv, new_idepth, HdiF):
         """makeCoarseDepthL0 on the device with the resident frame as the reference; returns pc_n per level"""

@@ -83,13 +83,11 @@ int dmv_ba_create(const dmv_ba_config* cfg, dmv_ba** out) {
   }
   if (cfg->device < 0 || cfg->device >= ndev) return set_error(DMV_ERR_INVALID, "device %d out of range (%d devices)", cfg->device, ndev);
   CK(cudaSetDevice(cfg->device));
-  {  // L2 -> DRAM fetch granularity: 32 B instead of the driver default 64 B.  The hot path gathers 16-byte texels at data-dependent addresses;
-     // with 64-byte fetches every missed 32-byte sector drags its neighbour along: measured 7.58 -> 5.69 MB DRAM reads per launch at C3 (1.38x ->
-     // 1.04x the algorithmic bytes, profiles/r02_a_l2fetch_*), no change in kernel time.  A device-wide hint; DMV_L2_FETCH=64|128 restores / widens it.
-    int g = 32;
-    if (const char* e = getenv("DMV_L2_FETCH")) g = atoi(e);
-    if (g == 32 || g == 64 || g == 128) { cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)g); cudaGetLastError(); }
-  }
+  // L2 -> DRAM fetch granularity: 32 B instead of the driver default 64 B.  The hot path gathers 16-byte texels at data-dependent addresses;
+  // with 64-byte fetches every missed 32-byte sector drags its neighbour along: measured 7.58 -> 5.69 MB DRAM reads per launch at C3 (1.38x ->
+  // 1.04x the algorithmic bytes, profiles/r02_a_l2fetch_*), no change in kernel time.  A device-wide hint.
+  cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, 32);
+  cudaGetLastError();
   dmv_ba* b = new dmv_ba();
   const int rc = ba_allocate(b, cfg);
   if (rc != DMV_OK) {  // e.g. out of device memory half-way: release what was allocated (the error message of the failing call is kept)
@@ -104,7 +102,6 @@ static int ba_allocate(dmv_ba* b, const dmv_ba_config* cfg) {
   b->cfg = *cfg;
   b->device = cfg->device;
   dmv_ba_default_params(&b->prm);
-  if (const char* e = getenv("DMV_NO_ZERO_COPY")) b->no_zero_copy = atoi(e) != 0;
   // chunk_points 16 / 32 force the shape; 0 = per window (dmv_ba_set_points): 16 while the window is one wave of 16-point chunks, else 32
   b->P_auto = !(cfg->chunk_points == 16 || cfg->chunk_points == 32);
   b->P = b->P_auto ? 16 : cfg->chunk_points;
@@ -406,7 +403,7 @@ static int enqueue_linearize(dmv_ba* b) {
   dmv_ba_fill_descriptor(b);
   dmv_ba_next_exchange(b);
   // the kernel writes the final blob into the pinned host mirror itself, unless a NCCL all-reduce still follows it
-  const bool zero_copy = !(b->nccl_comm && !b->xchg_on) && !b->no_zero_copy;
+  const bool zero_copy = !(b->nccl_comm && !b->xchg_on);
   double* hres = b->h_result[b->tent];
   hres[(size_t)b->N * b->N + b->N + (size_t)b->ntiles * 16 + (ACC_MISC - 1)] = 0.0;  // error flag: written by the device on a timeout only
   if (zero_copy) b->h_up->win.result_host = hres;

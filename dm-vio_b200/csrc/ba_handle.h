@@ -77,7 +77,6 @@ struct dmv_ba {
   std::vector<uint8_t> h_st_in;
   std::vector<float> h_en_in;
   bool st_in_clean = false;    // every existing residual's INPUT state on the device is IN with zero energy (dmv_ba_reset_oob becomes a flag flip)
-  bool no_zero_copy = false;   // DMV_NO_ZERO_COPY=1: D2H copy node instead of in-kernel writes to the pinned result (A/B experiment)
   bool timing = false;         // record CUDA events around the kernels of every call (dmv_ba_set_timing)
   int tent = 0;                // index of the tentative buffer set; committed = 1 - tent
   bool have_tentative = false, have_committed = false, have_adj = false, have_state = false;

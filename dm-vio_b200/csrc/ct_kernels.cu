@@ -31,71 +31,72 @@ struct CTParams {
   int w, h, n, lvl, want_gs;
 };
 
-// one reference point: CoarseTracker::calcRes (L399-483) + its row of calcGSSSE (L316-336); v[] = this point's contribution
-__device__ __forceinline__ void ct_eval_point(const CTParams& P, int i, const float* __restrict__ pc_u, const float* __restrict__ pc_v,
-                                              const float* __restrict__ pc_id, const float* __restrict__ pc_col, const float4* __restrict__ img,
-                                              float v[CT_NRED]) {
-#pragma unroll
-  for (int k = 0; k < CT_NRED; k++) v[k] = 0.f;
-  if (i < P.n) {
-    const float id = pc_id[i], x = pc_u[i], y = pc_v[i];
-    const float p0 = P.RKi[0] * x + P.RKi[1] * y + P.RKi[2] + P.t[0] * id;
-    const float p1 = P.RKi[3] * x + P.RKi[4] * y + P.RKi[5] + P.t[1] * id;
-    const float p2 = P.RKi[6] * x + P.RKi[7] * y + P.RKi[8] + P.t[2] * id;
-    const float u = p0 / p2, vv = p1 / p2;
-    const float Ku = P.fx * u + P.cx, Kv = P.fy * vv + P.cy;
-    const float new_idepth = id / p2;
-    if (P.lvl == 0 && (i & 31) == 0) {  // flow indicators (L416-447)
-      const float k0 = P.Ki[0] * x + P.Ki[1] * y + P.Ki[2], k1 = P.Ki[3] * x + P.Ki[4] * y + P.Ki[5], k2 = P.Ki[6] * x + P.Ki[7] * y + P.Ki[8];
-      const float T0 = k0 + P.t[0] * id, T1 = k1 + P.t[1] * id, T2 = k2 + P.t[2] * id;
-      const float M0 = k0 - P.t[0] * id, M1 = k1 - P.t[1] * id, M2 = k2 - P.t[2] * id;
-      const float q0 = P.RKi[0] * x + P.RKi[1] * y + P.RKi[2] - P.t[0] * id;
-      const float q1 = P.RKi[3] * x + P.RKi[4] * y + P.RKi[5] - P.t[1] * id;
-      const float q2 = P.RKi[6] * x + P.RKi[7] * y + P.RKi[8] - P.t[2] * id;
-      const float KuT = P.fx * (T0 / T2) + P.cx, KvT = P.fy * (T1 / T2) + P.cy;
-      const float KuT2 = P.fx * (M0 / M2) + P.cx, KvT2 = P.fy * (M1 / M2) + P.cy;
-      const float Ku3 = P.fx * (q0 / q2) + P.cx, Kv3 = P.fy * (q1 / q2) + P.cy;
-      v[49] = (KuT - x) * (KuT - x) + (KvT - y) * (KvT - y) + (KuT2 - x) * (KuT2 - x) + (KvT2 - y) * (KvT2 - y);
-      v[50] = (Ku - x) * (Ku - x) + (Kv - y) * (Kv - y) + (Ku3 - x) * (Ku3 - x) + (Kv3 - y) * (Kv3 - y);
-      v[51] = 2.f;
-    }
-    if (Ku > 2.f && Kv > 2.f && Ku < (float)(P.w - 3) && Kv < (float)(P.h - 3) && new_idepth > 0.f) {
-      const int ix = (int)Ku, iy = (int)Kv;
-      const float dx = Ku - ix, dy = Kv - iy, dxdy = dx * dy;
+// one reference point: CoarseTracker::calcRes (L399-483) + its row of calcGSSSE (L316-336), added into v[].  The 4 taps are gathered from
+// the level plane in global memory (SMEM = false) or from its copy staged in shared memory (SMEM = true).
+template <bool SMEM>
+__device__ __forceinline__ void ct_eval_point(const CTParams& P, int i, const float x, const float y, const float id, const float refColor,
+                                              const float4* __restrict__ img, float v[CT_NRED]) {
+  const float p0 = P.RKi[0] * x + P.RKi[1] * y + P.RKi[2] + P.t[0] * id;
+  const float p1 = P.RKi[3] * x + P.RKi[4] * y + P.RKi[5] + P.t[1] * id;
+  const float p2 = P.RKi[6] * x + P.RKi[7] * y + P.RKi[8] + P.t[2] * id;
+  const float u = p0 / p2, vv = p1 / p2;
+  const float Ku = P.fx * u + P.cx, Kv = P.fy * vv + P.cy;
+  const float new_idepth = id / p2;
+  if (P.lvl == 0 && (i & 31) == 0) {  // flow indicators (L416-447)
+    const float k0 = P.Ki[0] * x + P.Ki[1] * y + P.Ki[2], k1 = P.Ki[3] * x + P.Ki[4] * y + P.Ki[5], k2 = P.Ki[6] * x + P.Ki[7] * y + P.Ki[8];
+    const float T0 = k0 + P.t[0] * id, T1 = k1 + P.t[1] * id, T2 = k2 + P.t[2] * id;
+    const float M0 = k0 - P.t[0] * id, M1 = k1 - P.t[1] * id, M2 = k2 - P.t[2] * id;
+    const float q0 = P.RKi[0] * x + P.RKi[1] * y + P.RKi[2] - P.t[0] * id;
+    const float q1 = P.RKi[3] * x + P.RKi[4] * y + P.RKi[5] - P.t[1] * id;
+    const float q2 = P.RKi[6] * x + P.RKi[7] * y + P.RKi[8] - P.t[2] * id;
+    const float KuT = P.fx * (T0 / T2) + P.cx, KvT = P.fy * (T1 / T2) + P.cy;
+    const float KuT2 = P.fx * (M0 / M2) + P.cx, KvT2 = P.fy * (M1 / M2) + P.cy;
+    const float Ku3 = P.fx * (q0 / q2) + P.cx, Kv3 = P.fy * (q1 / q2) + P.cy;
+    v[49] += (KuT - x) * (KuT - x) + (KvT - y) * (KvT - y) + (KuT2 - x) * (KuT2 - x) + (KvT2 - y) * (KvT2 - y);
+    v[50] += (Ku - x) * (Ku - x) + (Kv - y) * (Kv - y) + (Ku3 - x) * (Ku3 - x) + (Kv3 - y) * (Kv3 - y);
+    v[51] += 2.f;
+  }
+  if (Ku > 2.f && Kv > 2.f && Ku < (float)(P.w - 3) && Kv < (float)(P.h - 3) && new_idepth > 0.f) {
+    const int ix = (int)Ku, iy = (int)Kv;
+    const float dx = Ku - ix, dy = Kv - iy, dxdy = dx * dy;
+    float4 tl, tr, bl, br;
+    if constexpr (SMEM) {
+      const float4* bp = img + iy * P.w + ix;
+      tl = bp[0]; tr = bp[1]; bl = bp[P.w]; br = bp[P.w + 1];
+    } else {
       const float4* bp = img + (size_t)iy * P.w + ix;
-      const float4 tl = __ldg(bp), tr = __ldg(bp + 1), bl = __ldg(bp + P.w), br = __ldg(bp + P.w + 1);
-      const float w11 = dxdy, w10 = dy - dxdy, w01 = dx - dxdy, w00 = 1 - dx - dy + dxdy;
-      const float h0 = w11 * br.x + w10 * bl.x + w01 * tr.x + w00 * tl.x;
-      const float h1 = w11 * br.y + w10 * bl.y + w01 * tr.y + w00 * tl.y;
-      const float h2 = w11 * br.z + w10 * bl.z + w01 * tr.z + w00 * tl.z;
-      if (isfinite(h0)) {
-        const float refColor = pc_col[i];
-        const float residual = h0 - (P.affa * refColor + P.affb);
-        const float ar = fabsf(residual);
-        const float hw = ar < P.huber ? 1.f : P.huber / ar;
-        if (ar > P.cutoff) {
-          v[45] = P.maxEnergy; v[46] = 1.f; v[47] = 1.f;
-        } else {
-          v[45] = hw * residual * residual * (2.f - hw); v[46] = 1.f; v[48] = 1.f;
-          if (P.want_gs) {  // calcGSSSE row (L316-336) and Accumulator9::updateSSE_eighted (MatrixAccumulators.h:L1091-1166)
-            const float gx = h1 * P.fx, gy = h2 * P.fy;
-            float J[9];
-            J[0] = new_idepth * gx;
-            J[1] = new_idepth * gy;
-            J[2] = 0.f - new_idepth * (u * gx + vv * gy);
-            J[3] = 0.f - ((u * vv) * gx + gy * (1.f + vv * vv));
-            J[4] = (u * vv) * gy + gx * (1.f + u * u);
-            J[5] = u * gy - vv * gx;
-            J[6] = P.a_gs * (P.b0 - refColor);
-            J[7] = -1.f;
-            J[8] = residual;
-            int e = 0;
+      tl = __ldg(bp); tr = __ldg(bp + 1); bl = __ldg(bp + P.w); br = __ldg(bp + P.w + 1);
+    }
+    const float w11 = dxdy, w10 = dy - dxdy, w01 = dx - dxdy, w00 = 1 - dx - dy + dxdy;
+    const float h0 = w11 * br.x + w10 * bl.x + w01 * tr.x + w00 * tl.x;
+    const float h1 = w11 * br.y + w10 * bl.y + w01 * tr.y + w00 * tl.y;
+    const float h2 = w11 * br.z + w10 * bl.z + w01 * tr.z + w00 * tl.z;
+    if (isfinite(h0)) {
+      const float residual = h0 - (P.affa * refColor + P.affb);
+      const float ar = fabsf(residual);
+      const float hw = ar < P.huber ? 1.f : P.huber / ar;
+      if (ar > P.cutoff) {
+        v[45] += P.maxEnergy; v[46] += 1.f; v[47] += 1.f;
+      } else {
+        v[45] += hw * residual * residual * (2.f - hw); v[46] += 1.f; v[48] += 1.f;
+        if (P.want_gs) {  // calcGSSSE row (L316-336) and Accumulator9::updateSSE_eighted (MatrixAccumulators.h:L1091-1166)
+          const float gx = h1 * P.fx, gy = h2 * P.fy;
+          float J[9];
+          J[0] = new_idepth * gx;
+          J[1] = new_idepth * gy;
+          J[2] = 0.f - new_idepth * (u * gx + vv * gy);
+          J[3] = 0.f - ((u * vv) * gx + gy * (1.f + vv * vv));
+          J[4] = (u * vv) * gy + gx * (1.f + u * u);
+          J[5] = u * gy - vv * gx;
+          J[6] = P.a_gs * (P.b0 - refColor);
+          J[7] = -1.f;
+          J[8] = residual;
+          int e = 0;
 #pragma unroll
-            for (int r = 0; r < 9; r++) {
-              const float Jw = J[r] * hw;
+          for (int r = 0; r < 9; r++) {
+            const float Jw = J[r] * hw;
 #pragma unroll
-              for (int c = r; c < 9; c++) v[e++] = Jw * J[c];
-            }
+            for (int c = r; c < 9; c++) v[e++] += Jw * J[c];
           }
         }
       }
@@ -153,7 +154,9 @@ __global__ void __launch_bounds__(CT_THREADS) ct_res_gs_kernel(CTParams P, const
                                                                unsigned int* __restrict__ ticket, double* __restrict__ out) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   float v[CT_NRED];
-  ct_eval_point(P, i, pc_u, pc_v, pc_id, pc_col, img, v);
+#pragma unroll
+  for (int k = 0; k < CT_NRED; k++) v[k] = 0.f;
+  if (i < P.n) ct_eval_point<false>(P, i, pc_u[i], pc_v[i], pc_id[i], pc_col[i], img, v);
   __shared__ float s_red[CT_THREADS / 32][CT_NRED];
   const double bs = ct_block_reduce(v, s_red);
   if (threadIdx.x < CT_NRED) partial[(size_t)blockIdx.x * CT_NRED + threadIdx.x] = bs;
@@ -177,17 +180,34 @@ __global__ void __launch_bounds__(CT_THREADS) ct_res_gs_kernel(CTParams P, const
   }
 }
 
-// ---------------------------------------------------------------------------------------------------------------------
-// ct_track_kernel — CoarseTracker::trackNewestCoarse (CoarseTracker.cpp:L539-770, visual-only branch L639-683) as ONE persistent
-// launch: the Levenberg-Marquardt loop over all pyramid levels runs on the device.  G = ceil(max_l n_l / 256) co-resident CTAs
-// (cooperative launch); one evaluation = every CTA evaluates its points (calcRes + calcGSSSE row, as ct_res_gs_kernel), per-CTA
-// fp64 partials, a grid barrier, then EVERY CTA folds the partials in CTA order and its thread 0 advances the same scalar state
-// machine in double (8x8 LDLT, SE3 exp, accept/reject, level schedule) - identical inputs, identical decisions, so no second
-// barrier and no broadcast.  Replaces ~21 launch + sync round trips per frame by one launch.
-// ---------------------------------------------------------------------------------------------------------------------
+// Vec6 of calcRes (L508-516) and H, b of calcGSSSE (L341-355) from the 53 folded sums o[]: output k < 64 is H[k], 64 <= k < 72 is
+// b[k - 64], k == 72 is all of res6.  H and b are divided by the 4-padded warped count (buf_warped_n), then scaled by SCALE_A / SCALE_B.
+__host__ __device__ __forceinline__ void ct_finish(const double* o, int k, double* res6, double* H, double* b) {
+  const int npad = ((int)o[48] + 3) & ~3;
+  const double inv = (double)(1.0f / (float)npad);
+  if (k < 72) {
+    const int r = (k < 64) ? (k >> 3) : (k - 64), c = (k < 64) ? (k & 7) : 8;   // c = 8: the b column of the 9x9 accumulator
+    const int lo = r < c ? r : c, hi = r < c ? c : r;
+    const int e = lo * 9 - (lo * (lo - 1)) / 2 + (hi - lo);     // upper-triangular index of the 9x9 accumulator
+    const double scr = (r == 6) ? 10.0 : (r == 7 ? 1000.0 : 1.0);
+    if (k < 64) {
+      const double scc = (c == 6) ? 10.0 : (c == 7 ? 1000.0 : 1.0);
+      H[k] = o[e] * inv * scr * scc;
+    } else {
+      b[r] = o[e] * inv * scr;
+    }
+  } else if (k == 72) {
+    res6[0] = o[45]; res6[1] = o[46];
+    res6[2] = (double)((float)o[49] / ((float)o[51] + 0.1f));
+    res6[3] = 0;
+    res6[4] = (double)((float)o[50] / ((float)o[51] + 0.1f));
+    res6[5] = (double)((float)o[47] / (float)o[46]);
+  }
+}
+
 constexpr int CT_L = DMV_MAX_PYR_LEVELS;
 struct CTTrack {
-  int levels, coarsest, G;
+  int coarsest;
   int n[CT_L], w[CT_L], h[CT_L];
   float fx[CT_L], fy[CT_L], cx[CT_L], cy[CT_L];
   float Ki[CT_L][9];
@@ -198,9 +218,7 @@ struct CTTrack {
   float ref_exposure, new_exposure;
   float huber, cutoffTH, affModeA, affModeB;
   double minRes[5];
-  double* partial;               // [2][G][CT_NRED]
-  unsigned int* bar;             // monotonic arrival counter, zero at launch
-  double* out;                   // pinned host: R[9] t[3] a b lastResiduals[5] flow[3] good iterations evaluations status
+  double* out;                   // pinned host: R[9] t[3] a b lastResiduals[5] flow[3] good iterations evaluations status point-evaluations
 };
 
 struct CTLM {  // the scalar state of trackNewestCoarse, one copy per CTA (shared memory), advanced by thread 0
@@ -219,50 +237,17 @@ struct CTLM {  // the scalar state of trackNewestCoarse, one copy per CTA (share
 };
 enum { CT_PH_INIT = 0, CT_PH_LM = 1 };
 
-// Hl.ldlt().solve(-b) for the 8x8 system (L639-665): plain LDL^T (ct_factor_warp / ct_propose_post below).  A parameter that is not
-// optimised (setting_affineOptModeA/B < 0: the reference solves the 6x6 / 7x7 sub-system) is padded with an identity row/column and a zero
-// right-hand side: the extra terms are exact zeros, the other components come out bit-identical.
-// operands of calcRes for a pose (CoarseTracker.cpp:L377-379): RKi = R.cast<float>() * Ki[lvl], t.cast<float>(), affLL.cast<float>()
-__device__ __forceinline__ void ct_request(const CTTrack& T, CTLM& S, const double R[9], const double t[3], double a, double b) {
-  (void)T; (void)R; (void)t; (void)a; (void)b;
-  S.need_request = 1;   // evaluate at the current pose: the warp forms the operands (ct_pose_request_warp)
-}
-// Vec6 of calcRes (L508-516) and H, b of calcGSSSE (L341-355) from the 53 folded sums, one output per thread (tid < 78)
-__device__ __forceinline__ void ct_finish_parallel(const double* o, double* res6, double* H, double* b, int tid) {
-  const int npad = ((int)o[48] + 3) & ~3;
-  const double inv = (double)(1.0f / (float)npad);
-  if (tid < 72) {
-    const int r = tid >> 3, c = (tid < 64) ? (tid & 7) : 8;   // tid 64..71: r = 8 -> handled below as the b column
-    const int rr = (tid < 64) ? r : (tid - 64);
-    const int lo = rr < c ? rr : c, hi = rr < c ? c : rr;
-    const int e = lo * 9 - (lo * (lo - 1)) / 2 + (hi - lo);     // upper-triangular index of the 9x9 accumulator
-    const double scr = (rr == 6) ? 10.0 : (rr == 7 ? 1000.0 : 1.0);
-    if (tid < 64) {
-      const double scc = (c == 6) ? 10.0 : (c == 7 ? 1000.0 : 1.0);
-      H[rr * 8 + c] = o[e] * inv * scr * scc;
-    } else {
-      b[rr] = o[e] * inv * scr;
-    }
-  } else if (tid == 72) {
-    res6[0] = o[45]; res6[1] = o[46];
-    res6[2] = (double)((float)o[49] / ((float)o[51] + 0.1f));
-    res6[3] = 0;
-    res6[4] = (double)((float)o[50] / ((float)o[51] + 0.1f));
-    res6[5] = (double)((float)o[47] / (float)o[46]);
-  }
-}
-__device__ void ct_begin_level(const CTTrack& T, CTLM& S) {
+__device__ void ct_begin_level(CTLM& S) {
   S.rep = 1.f;
   S.phase = CT_PH_INIT;
-  ct_request(T, S, S.R, S.t, S.a, S.b);
+  S.need_request = 1;
 }
-// one LM trial step from the current linearisation (L605-683), in three parts: lane 0 sets up the damped system, the WARP factorises it
+// one LM trial step from the current linearisation (L605-683), in three parts: the warp sets up the damped system and factorises it
 // (row i of L in lane i: the 8^3/3 multiply-adds and the 28 divisions of the scalar version collapse to 8 dependent column steps), lane 0
 // substitutes and updates the pose.  Every element sees the same operations in the same order as the scalar LDL^T: bit-identical result.
-__device__ void ct_propose_pre(const CTTrack& T, CTLM& S) {  // lane 0: bookkeeping only; the damped system is built by the warp (ct_build_system_warp)
-  S.iterations++;
-  S.need_solve = 1;
-}
+// Hl.ldlt().solve(-b) for the 8x8 system (L639-665): plain LDL^T.  A parameter that is not optimised (setting_affineOptModeA/B < 0: the
+// reference solves the 6x6 / 7x7 sub-system) is padded with an identity row/column and a zero right-hand side: the extra terms are exact
+// zeros, the other components come out bit-identical.
 __device__ __forceinline__ void ct_build_system_warp(const CTTrack& T, CTLM& S) {
   const int lane = threadIdx.x & 31;
   const double* Hc = S.H[S.cur];
@@ -353,7 +338,7 @@ __device__ void ct_propose_post(const CTTrack& T, CTLM& S) {
   S.need_request = 2;   // evaluate at the candidate exp(incs) * (R, t)
 }
 // SE3::exp(incs) * (R, t) -> (Rn, tn) and the operands of the next calcRes, spread over the lanes of warp 0: every output element is formed
-// by exactly the expression of the scalar code (ct_se3_exp_mul / ct_request), only by a different lane.
+// by exactly the expression of the scalar code, only by a different lane.
 __device__ __forceinline__ void ct_pose_request_warp(const CTTrack& T, CTLM& S, const bool from_candidate) {
   const int lane = threadIdx.x & 31;
   if (from_candidate) {
@@ -404,15 +389,13 @@ __device__ __forceinline__ void ct_pose_request_warp(const CTTrack& T, CTLM& S, 
     S.pevals += (double)T.n[S.lvl];
   }
 }
-// the scalar state machine step, executed by warp 0 of every CTA
-__device__ __forceinline__ void ct_advance_warp(const CTTrack& T, CTLM& S);
 __device__ void ct_end_level(const CTTrack& T, CTLM& S) {  // L722-745
   const int lvl = S.lvl;
   const double* resOld = S.res[S.cur];
   S.lastResiduals[lvl] = sqrtf((float)(resOld[0] / resOld[1]));
   S.flow[0] = resOld[2]; S.flow[1] = resOld[3]; S.flow[2] = resOld[4];
   if (isnan(S.lastResiduals[lvl]) || S.lastResiduals[lvl] > 1.5 * T.minRes[lvl]) { S.done = 1; S.good = 0; S.status = 2; return; }
-  if (S.rep > 1 && !S.haveRepeated) { S.haveRepeated = 1; ct_begin_level(T, S); return; }  // lvl++ ; continue  => the same level again
+  if (S.rep > 1 && !S.haveRepeated) { S.haveRepeated = 1; ct_begin_level(S); return; }  // lvl++ ; continue  => the same level again
   S.lvl = lvl - 1;
   if (S.lvl < 0) {  // L747-769
     S.done = 1;
@@ -427,20 +410,22 @@ __device__ void ct_end_level(const CTTrack& T, CTLM& S) {  // L722-745
     S.good = good ? 1 : 0;
     return;
   }
-  ct_begin_level(T, S);
+  ct_begin_level(S);
 }
-// thread 0: the evaluation that just finished sits in S.res/H/bb[cur^1] (ct_finish_parallel); decide what to evaluate next
+// thread 0: the evaluation that just finished sits in S.res/H/bb[cur^1] (ct_finish); decide what to evaluate next: the same pose again
+// (need_request = 1), an LM step from the current linearisation (need_solve), or the next level
 __device__ void ct_advance(const CTTrack& T, CTLM& S) {
   const int maxIterations[5] = {10, 20, 50, 50, 50};
   const int nw = S.cur ^ 1;
   const double* res = S.res[nw];
   if (S.phase == CT_PH_INIT) {  // L566-578: first evaluation of a level, cutoff doubling while too many residuals saturate
     S.cur = nw;                 // this evaluation becomes the current linearisation (resOld, H, b)
-    if (res[5] > 0.6 && (S.rep < 50 || res[5] > 0.99)) { S.rep *= 2; ct_request(T, S, S.R, S.t, S.a, S.b); return; }
+    if (res[5] > 0.6 && (S.rep < 50 || res[5] > 0.99)) { S.rep *= 2; S.need_request = 1; return; }
     S.lambda = 0.01f;
     S.iteration = 0;
     if (S.iteration >= maxIterations[S.lvl]) { ct_end_level(T, S); return; }
-    ct_propose_pre(T, S);
+    S.iterations++;
+    S.need_solve = 1;
     return;
   }
   // CT_PH_LM: accept / reject (L686-716)
@@ -461,8 +446,10 @@ __device__ void ct_advance(const CTTrack& T, CTLM& S) {
   incNorm = sqrt(incNorm);
   S.iteration++;
   if (!(incNorm > 1e-3) || S.iteration >= maxIterations[S.lvl]) { ct_end_level(T, S); return; }
-  ct_propose_pre(T, S);
+  S.iterations++;
+  S.need_solve = 1;
 }
+// the scalar state machine step, executed by warp 0 of every CTA
 __device__ __forceinline__ void ct_advance_warp(const CTTrack& T, CTLM& S) {
   const int lane = threadIdx.x & 31;
   if (lane == 0) { S.need_request = 0; ct_advance(T, S); }
@@ -478,92 +465,21 @@ __device__ __forceinline__ void ct_advance_warp(const CTTrack& T, CTLM& S) {
   if (S.need_request) ct_pose_request_warp(T, S, S.need_request == 2);
 }
 
-__global__ void __launch_bounds__(CT_THREADS) ct_track_kernel(const __grid_constant__ CTTrack T) {
-  __shared__ float s_red[CT_THREADS / 32][CT_NRED];
-  __shared__ double s_sum[CT_NRED];
-  __shared__ double s_q[4][CT_NRED];
-  __shared__ CTLM S;
-  const int tid = threadIdx.x;
-  const int G = T.G;
-  unsigned int epoch = 0;
-  int par = 0;
-  if (tid == 0) {
-    for (int i = 0; i < 9; i++) S.R[i] = T.R0[i];
-    for (int i = 0; i < 3; i++) S.t[i] = T.t0[i];
-    S.a = T.a0; S.b = T.b0;
-    for (int i = 0; i < 5; i++) S.lastResiduals[i] = __longlong_as_double(0x7ff8000000000000ll);  // NAN
-    for (int i = 0; i < 3; i++) S.flow[i] = 1000;
-    S.haveRepeated = 0; S.iterations = 0; S.evaluations = 0; S.done = 0; S.good = 0; S.status = 0; S.cur = 0; S.need_solve = 0; S.pevals = 0;
-    S.lvl = T.coarsest;
-    ct_begin_level(T, S);
-  }
-  __syncthreads();
-  if (tid < 32) ct_pose_request_warp(T, S, false);
-  __syncthreads();
-  while (!S.done) {
-    // ---- one evaluation: calcRes + calcGSSSE at the requested pose
-    CTParams P;
-    const int l = S.lvl;
-#pragma unroll
-    for (int i = 0; i < 9; i++) { P.RKi[i] = S.RKi[i]; P.Ki[i] = T.Ki[l][i]; }
-#pragma unroll
-    for (int i = 0; i < 3; i++) P.t[i] = S.tf[i];
-    P.fx = T.fx[l]; P.fy = T.fy[l]; P.cx = T.cx[l]; P.cy = T.cy[l];
-    P.affa = S.affLL[0]; P.affb = S.affLL[1]; P.a_gs = S.affLL[0]; P.b0 = (float)T.ref_b;
-    P.cutoff = S.cutoff; P.huber = T.huber; P.maxEnergy = 2 * T.huber * S.cutoff - T.huber * T.huber;
-    P.w = T.w[l]; P.h = T.h[l]; P.n = T.n[l]; P.lvl = l; P.want_gs = 1;
-    float v[CT_NRED];
-    ct_eval_point(P, blockIdx.x * CT_THREADS + tid, T.u[l], T.v[l], T.id[l], T.col[l], T.img[l], v);
-    const double bs = ct_block_reduce(v, s_red);
-    if (tid < CT_NRED) T.partial[((size_t)par * G + blockIdx.x) * CT_NRED + tid] = bs;
-    // ---- grid barrier (all G CTAs are co-resident: cooperative launch)
-    __syncthreads();
-    if (tid == 0) {
-      __threadfence();
-      epoch += (unsigned)G;
-      atomicAdd(T.bar, 1u);
-      unsigned long long t_start;
-      asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t_start));
-      while (*((volatile unsigned int*)T.bar) < epoch) {
-        unsigned long long t_now;
-        asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t_now));
-        if (t_now - t_start > 200000000ull) { S.done = 1; S.good = 0; S.status = 1; break; }  // 0.2 s: never hang the GPU on a lost CTA
-      }
-      __threadfence();
-    }
-    __syncthreads();
-    if (S.status == 1) break;
-    // ---- every CTA folds the partials in CTA order (bit-identical sums everywhere) and advances the same state machine
-    ct_fold(T.partial + (size_t)par * G * CT_NRED, G, s_q, s_sum);
-    par ^= 1;
-    __syncthreads();
-    ct_finish_parallel(s_sum, S.res[S.cur ^ 1], S.H[S.cur ^ 1], S.bb[S.cur ^ 1], tid);
-    __syncthreads();
-    if (tid < 32) ct_advance_warp(T, S);
-    __syncthreads();
-  }
-  if (blockIdx.x == 0 && tid == 0) {
-    double* o = T.out;
-    const bool ok = (S.status == 0);
-    for (int i = 0; i < 9; i++) o[i] = ok ? S.R[i] : T.R0[i];
-    for (int i = 0; i < 3; i++) o[9 + i] = ok ? S.t[i] : T.t0[i];
-    o[12] = ok ? S.a : T.a0; o[13] = ok ? S.b : T.b0;
-    for (int i = 0; i < 5; i++) o[14 + i] = S.lastResiduals[i];
-    for (int i = 0; i < 3; i++) o[19 + i] = S.flow[i];
-    o[22] = S.good; o[23] = S.iterations; o[24] = S.evaluations; o[25] = S.status; o[26] = S.pevals;
-  }
-}
-
 // ---------------------------------------------------------------------------------------------------------------------
-// ct_track_cluster_kernel — the same trackNewestCoarse state machine on ONE THREAD-BLOCK CLUSTER (sm_90+ hardware feature):
+// ct_track_cluster_kernel — CoarseTracker::trackNewestCoarse (CoarseTracker.cpp:L539-770, visual-only branch L639-683) as ONE persistent
+// launch on ONE THREAD-BLOCK CLUSTER (sm_90+ hardware feature): the Levenberg-Marquardt loop over all pyramid levels runs on the device and
+// replaces ~21 launch + sync round trips per frame.  One evaluation = every CTA evaluates its points (calcRes + calcGSSSE row, the same
+// ct_eval_point as ct_res_gs_kernel), then EVERY CTA folds the cluster's partials in rank order and its warp 0 advances the same scalar
+// state machine in double (8x8 LDLT, SE3 exp, accept/reject, level schedule): identical inputs, identical decisions, so no second
+// barrier and no broadcast.
 //   * the CTAs of the cluster exchange their fp64 partials through DISTRIBUTED SHARED MEMORY (st.shared::cluster into every peer's
 //     slot) and meet at the hardware cluster barrier (barrier.cluster.arrive/wait): no global-memory partials, no atomics, no spinning
-//     on an L2 counter — the per-evaluation synchronisation of the 39-CTA grid version (~4 us) shrinks to a few hundred ns;
+//     on an L2 counter, a few hundred ns per evaluation;
 //   * pyramid levels whose float4 plane fits in shared memory (80x60 at 640x480: 76.8 KB; 64x64 at 512^2; 40x30) are staged ONCE per
 //     level by TMA (cp.async.bulk.tensor.2d, multicast to every CTA of the cluster, completion on an mbarrier) and every Levenberg-
 //     Marquardt evaluation of that level gathers its 4 taps per point from shared memory instead of L2;
-//   * the block reduction of the 53 sums per point is a transposing butterfly (62 shuffles per warp instead of 265).
-// Every CTA folds the cluster's partials in rank order and advances the same scalar state machine: identical decisions everywhere.
+//   * the block reduction of the 53 sums per point is a transposing butterfly (62 shuffles per warp instead of 265);
+//   * each thread keeps CTC_SLOTS reference points of the level in registers and streams the rest, so any point count is tracked.
 // A sequential LM chain is latency-bound: fewer, closer SMs with a hardware barrier beat a chip-wide software barrier (DESIGN.md §5).
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int CTC_THREADS = 512;
@@ -588,76 +504,6 @@ __device__ __forceinline__ void ctc_cluster_sync() {
 }
 __device__ __forceinline__ unsigned ctc_smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 
-// one reference point against a plane in SHARED memory (same arithmetic as ct_eval_point; the taps come from the staged copy)
-template <bool SMEM>
-__device__ __forceinline__ void ctc_eval_accumulate(const CTParams& P, int i, const float x, const float y, const float id, const float refColor,
-                                                    const float4* __restrict__ img, const float4* plane_s, float v[CT_NRED]) {
-  const float p0 = P.RKi[0] * x + P.RKi[1] * y + P.RKi[2] + P.t[0] * id;
-  const float p1 = P.RKi[3] * x + P.RKi[4] * y + P.RKi[5] + P.t[1] * id;
-  const float p2 = P.RKi[6] * x + P.RKi[7] * y + P.RKi[8] + P.t[2] * id;
-  const float u = p0 / p2, vv = p1 / p2;
-  const float Ku = P.fx * u + P.cx, Kv = P.fy * vv + P.cy;
-  const float new_idepth = id / p2;
-  if (P.lvl == 0 && (i & 31) == 0) {  // flow indicators (CoarseTracker.cpp:L416-447)
-    const float k0 = P.Ki[0] * x + P.Ki[1] * y + P.Ki[2], k1 = P.Ki[3] * x + P.Ki[4] * y + P.Ki[5], k2 = P.Ki[6] * x + P.Ki[7] * y + P.Ki[8];
-    const float T0 = k0 + P.t[0] * id, T1 = k1 + P.t[1] * id, T2 = k2 + P.t[2] * id;
-    const float M0 = k0 - P.t[0] * id, M1 = k1 - P.t[1] * id, M2 = k2 - P.t[2] * id;
-    const float q0 = P.RKi[0] * x + P.RKi[1] * y + P.RKi[2] - P.t[0] * id;
-    const float q1 = P.RKi[3] * x + P.RKi[4] * y + P.RKi[5] - P.t[1] * id;
-    const float q2 = P.RKi[6] * x + P.RKi[7] * y + P.RKi[8] - P.t[2] * id;
-    const float KuT = P.fx * (T0 / T2) + P.cx, KvT = P.fy * (T1 / T2) + P.cy;
-    const float KuT2 = P.fx * (M0 / M2) + P.cx, KvT2 = P.fy * (M1 / M2) + P.cy;
-    const float Ku3 = P.fx * (q0 / q2) + P.cx, Kv3 = P.fy * (q1 / q2) + P.cy;
-    v[49] += (KuT - x) * (KuT - x) + (KvT - y) * (KvT - y) + (KuT2 - x) * (KuT2 - x) + (KvT2 - y) * (KvT2 - y);
-    v[50] += (Ku - x) * (Ku - x) + (Kv - y) * (Kv - y) + (Ku3 - x) * (Ku3 - x) + (Kv3 - y) * (Kv3 - y);
-    v[51] += 2.f;
-  }
-  if (Ku > 2.f && Kv > 2.f && Ku < (float)(P.w - 3) && Kv < (float)(P.h - 3) && new_idepth > 0.f) {
-    const int ix = (int)Ku, iy = (int)Kv;
-    const float dx = Ku - ix, dy = Kv - iy, dxdy = dx * dy;
-    float4 tl, tr, bl, br;
-    if constexpr (SMEM) {
-      const float4* bp = plane_s + iy * P.w + ix;
-      tl = bp[0]; tr = bp[1]; bl = bp[P.w]; br = bp[P.w + 1];
-    } else {
-      const float4* bp = img + (size_t)iy * P.w + ix;
-      tl = __ldg(bp); tr = __ldg(bp + 1); bl = __ldg(bp + P.w); br = __ldg(bp + P.w + 1);
-    }
-    const float w11 = dxdy, w10 = dy - dxdy, w01 = dx - dxdy, w00 = 1 - dx - dy + dxdy;
-    const float h0 = w11 * br.x + w10 * bl.x + w01 * tr.x + w00 * tl.x;
-    const float h1 = w11 * br.y + w10 * bl.y + w01 * tr.y + w00 * tl.y;
-    const float h2 = w11 * br.z + w10 * bl.z + w01 * tr.z + w00 * tl.z;
-    if (isfinite(h0)) {
-      const float residual = h0 - (P.affa * refColor + P.affb);
-      const float ar = fabsf(residual);
-      const float hw = ar < P.huber ? 1.f : P.huber / ar;
-      if (ar > P.cutoff) {
-        v[45] += P.maxEnergy; v[46] += 1.f; v[47] += 1.f;
-      } else {
-        v[45] += hw * residual * residual * (2.f - hw); v[46] += 1.f; v[48] += 1.f;
-        const float gx = h1 * P.fx, gy = h2 * P.fy;
-        float J[9];
-        J[0] = new_idepth * gx;
-        J[1] = new_idepth * gy;
-        J[2] = 0.f - new_idepth * (u * gx + vv * gy);
-        J[3] = 0.f - ((u * vv) * gx + gy * (1.f + vv * vv));
-        J[4] = (u * vv) * gy + gx * (1.f + u * u);
-        J[5] = u * gy - vv * gx;
-        J[6] = P.a_gs * (P.b0 - refColor);
-        J[7] = -1.f;
-        J[8] = residual;
-        int e = 0;
-#pragma unroll
-        for (int r = 0; r < 9; r++) {
-          const float Jw = J[r] * hw;
-#pragma unroll
-          for (int c = r; c < 9; c++) v[e++] += Jw * J[c];
-        }
-      }
-    }
-  }
-}
-
 __global__ void __launch_bounds__(CTC_THREADS, 1) ct_track_cluster_kernel(const __grid_constant__ CTTrack T, const __grid_constant__ CTMaps maps) {
   extern __shared__ __align__(128) unsigned char ctc_raw[];
   CTCSmem& M = *reinterpret_cast<CTCSmem*>(ctc_raw);
@@ -675,7 +521,7 @@ __global__ void __launch_bounds__(CTC_THREADS, 1) ct_track_cluster_kernel(const 
     for (int i = 0; i < 3; i++) S.flow[i] = 1000;
     S.haveRepeated = 0; S.iterations = 0; S.evaluations = 0; S.done = 0; S.good = 0; S.status = 0; S.cur = 0; S.need_solve = 0; S.pevals = 0;
     S.lvl = T.coarsest;
-    ct_begin_level(T, S);
+    ct_begin_level(S);
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(ctc_smem_u32(&M.mbar)) : "memory");
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -734,13 +580,13 @@ __global__ void __launch_bounds__(CTC_THREADS, 1) ct_track_cluster_kernel(const 
     for (int k = 0; k < CTC_SLOTS; k++) {
       const int i = first + k * stride;
       if (i < P.n) {
-        if (fits) ctc_eval_accumulate<true>(P, i, pts[k].x, pts[k].y, pts[k].z, pts[k].w, T.img[l], reinterpret_cast<const float4*>(M.plane), v);
-        else ctc_eval_accumulate<false>(P, i, pts[k].x, pts[k].y, pts[k].z, pts[k].w, T.img[l], nullptr, v);
+        if (fits) ct_eval_point<true>(P, i, pts[k].x, pts[k].y, pts[k].z, pts[k].w, reinterpret_cast<const float4*>(M.plane), v);
+        else ct_eval_point<false>(P, i, pts[k].x, pts[k].y, pts[k].z, pts[k].w, T.img[l], v);
       }
     }
     for (int i = first + CTC_SLOTS * stride; i < P.n; i += stride) {  // more points than register slots: stream the rest
-      if (fits) ctc_eval_accumulate<true>(P, i, __ldg(T.u[l] + i), __ldg(T.v[l] + i), __ldg(T.id[l] + i), __ldg(T.col[l] + i), T.img[l], reinterpret_cast<const float4*>(M.plane), v);
-      else ctc_eval_accumulate<false>(P, i, __ldg(T.u[l] + i), __ldg(T.v[l] + i), __ldg(T.id[l] + i), __ldg(T.col[l] + i), T.img[l], nullptr, v);
+      if (fits) ct_eval_point<true>(P, i, __ldg(T.u[l] + i), __ldg(T.v[l] + i), __ldg(T.id[l] + i), __ldg(T.col[l] + i), reinterpret_cast<const float4*>(M.plane), v);
+      else ct_eval_point<false>(P, i, __ldg(T.u[l] + i), __ldg(T.v[l] + i), __ldg(T.id[l] + i), __ldg(T.col[l] + i), T.img[l], v);
     }
     // ---- warp: transposing butterfly, lane L ends with the warp sums of entries 2L, 2L+1
     {
@@ -778,17 +624,18 @@ __global__ void __launch_bounds__(CTC_THREADS, 1) ct_track_cluster_kernel(const 
     }
     par ^= 1;
     __syncthreads();
-    ct_finish_parallel(M.s_sum, S.res[S.cur ^ 1], S.H[S.cur ^ 1], S.bb[S.cur ^ 1], tid);
+    ct_finish(M.s_sum, tid, S.res[S.cur ^ 1], S.H[S.cur ^ 1], S.bb[S.cur ^ 1]);
     __syncthreads();
     if (tid < 32) ct_advance_warp(T, S);
     __syncthreads();
   }
   ctc_cluster_sync();  // nobody leaves while a peer may still write into its shared memory
-  if (rank == 0 && tid == 0) {
+  if (rank == 0 && tid == 0) {  // an aborted track (status 2) returns the input pose and affine parameters, like the reference's early return
     double* o = T.out;
-    for (int i = 0; i < 9; i++) o[i] = S.R[i];
-    for (int i = 0; i < 3; i++) o[9 + i] = S.t[i];
-    o[12] = S.a; o[13] = S.b;
+    const bool ok = (S.status == 0);
+    for (int i = 0; i < 9; i++) o[i] = ok ? S.R[i] : T.R0[i];
+    for (int i = 0; i < 3; i++) o[9 + i] = ok ? S.t[i] : T.t0[i];
+    o[12] = ok ? S.a : T.a0; o[13] = ok ? S.b : T.b0;
     for (int i = 0; i < 5; i++) o[14 + i] = S.lastResiduals[i];
     for (int i = 0; i < 3; i++) o[19 + i] = S.flow[i];
     o[22] = S.good; o[23] = S.iterations; o[24] = S.evaluations; o[25] = S.status; o[26] = S.pevals;
@@ -841,7 +688,6 @@ struct dmv_ct {
   int n[DMV_MAX_PYR_LEVELS];
   double* d_partial = nullptr;
   unsigned int* d_ticket = nullptr;
-  unsigned int* d_bar = nullptr;   // grid-barrier counter of ct_track_kernel
   double* d_out = nullptr;
   double* h_out = nullptr;
   float* h_scratch = nullptr;
@@ -852,7 +698,7 @@ struct dmv_ct {
   float* h_ip = nullptr;
   int ip_cap = 0;
   float huber = 9.f;
-  int cluster_size = 0;        // CTAs of ct_track_cluster_kernel's cluster (0 = not probed yet, -1 = unavailable: grid version)
+  int cluster_size = 0;        // CTAs of ct_track_cluster_kernel's cluster (0 = not probed yet, -1 = no TMA descriptors, -2 = no cluster fits)
   CTMaps* maps = nullptr;      // TMA descriptors of the level planes (host copy; passed as a kernel parameter)
   long long launches = 0;
   float last_ms[4] = {0, 0, 0, 0};
@@ -908,8 +754,7 @@ static int ct_allocate(dmv_ct* c, const dmv_ct_config* cfg) {
   const size_t npx0 = (size_t)cfg->w * cfg->h;
   CK(cudaMalloc(&c->d_stage, npx0 * 3 * sizeof(float)));
   const int maxBlocks = (cfg->max_points + CT_THREADS - 1) / CT_THREADS;
-  CK(cudaMalloc(&c->d_partial, sizeof(double) * CT_NRED * maxBlocks * 2));  // x2: ct_track_kernel double-buffers the per-CTA partials
-  CK(cudaMalloc(&c->d_bar, sizeof(unsigned int)));
+  CK(cudaMalloc(&c->d_partial, sizeof(double) * CT_NRED * maxBlocks));
   CK(cudaMalloc(&c->d_ticket, sizeof(unsigned int)));
   CK(cudaMemset(c->d_ticket, 0, sizeof(unsigned int)));
   CK(cudaMalloc(&c->d_out, sizeof(double) * 64));
@@ -925,7 +770,7 @@ int dmv_ct_destroy(dmv_ct* c) {
   for (int l = 0; l < DMV_MAX_PYR_LEVELS; l++) {
     cudaFree(c->d_img[l]); cudaFree(c->d_gray[l]); cudaFree(c->d_u[l]); cudaFree(c->d_v[l]); cudaFree(c->d_id[l]); cudaFree(c->d_col[l]);
   }
-  cudaFree(c->d_stage); cudaFree(c->d_partial); cudaFree(c->d_ticket); cudaFree(c->d_bar); cudaFree(c->d_out);
+  cudaFree(c->d_stage); cudaFree(c->d_partial); cudaFree(c->d_ticket); cudaFree(c->d_out);
   cudaFreeHost(c->h_out); cudaFreeHost(c->h_scratch); cudaFree(c->d_ip); cudaFreeHost(c->h_ip);
   for (int l = 0; l < DMV_MAX_PYR_LEVELS; l++) { cudaFree(c->cd_idepth[l]); cudaFree(c->cd_ws[l]); cudaFree(c->cd_ws2[l]); }
   cudaFree(c->cd_rowcnt); cudaFree(c->cd_rowoff); cudaFreeHost(c->cd_totals);
@@ -1036,28 +881,8 @@ int dmv_ct_calc_res_gs(dmv_ct* c, int l, const float RKi[9], const float t[3], c
   c->staging_busy = false;
   if (c->timing) cudaEventElapsedTime(&c->last_ms[0], c->ev[0], c->ev[1]);
   const double* o = c->h_out;
-  const double E = o[45], nE = o[46], nSat = o[47], nW = o[48];
-  res6[0] = E;
-  res6[1] = nE;
-  res6[2] = (double)((float)o[49] / ((float)o[51] + 0.1f));
-  res6[3] = 0;
-  res6[4] = (double)((float)o[50] / ((float)o[51] + 0.1f));
-  res6[5] = (double)((float)nSat / (float)nE);
-  const int npad = ((int)nW + 3) & ~3;
-  if (n_warped) *n_warped = npad;
-  if (want_gs) {
-    // acc.H (9x9) -> H_out = H[0:8,0:8] * (1/n), b_out = H[0:8,8] * (1/n), then SCALE_* (CoarseTracker.cpp:L341-355)
-    double M[9][9];
-    int e = 0;
-    for (int r = 0; r < 9; r++)
-      for (int cc = r; cc < 9; cc++) { M[r][cc] = M[cc][r] = o[e]; e++; }
-    const double inv = (double)(1.0f / (float)npad);
-    const double sc[8] = {1, 1, 1, 1, 1, 1, 10.0, 1000.0};  // SCALE_XI_ROT/TRANS = 1, SCALE_A, SCALE_B
-    for (int r = 0; r < 8; r++) {
-      for (int cc = 0; cc < 8; cc++) H[r * 8 + cc] = M[r][cc] * inv * sc[r] * sc[cc];
-      b[r] = M[r][8] * inv * sc[r];
-    }
-  }
+  for (int k = want_gs ? 0 : 72; k <= 72; k++) ct_finish(o, k, res6, H, b);
+  if (n_warped) *n_warped = ((int)o[48] + 3) & ~3;
   return DMV_OK;
 }
 
@@ -1089,15 +914,14 @@ static int ct_make_tensor_maps(dmv_ct* c) {
   return DMV_OK;
 }
 
-// CoarseTracker::trackNewestCoarse (CoarseTracker.cpp:L539-770, visual-only branch) in one persistent launch
+// CoarseTracker::trackNewestCoarse (CoarseTracker.cpp:L539-770, visual-only branch) in one persistent cluster launch
 int dmv_ct_track(dmv_ct* c, const dmv_ct_track_args* in, dmv_ct_track_result* out) {
   if (!c || !in || !out) return set_error(DMV_ERR_INVALID, "null argument");
   if (in->coarsestLvl < 0 || in->coarsestLvl >= c->cfg.levels || in->coarsestLvl >= 5) return set_error(DMV_ERR_INVALID, "coarsestLvl out of range");
   CK(cudaSetDevice(c->device));
   CTTrack T;
   std::memset(&T, 0, sizeof(T));
-  T.levels = c->cfg.levels; T.coarsest = in->coarsestLvl;
-  int maxn = 1;
+  T.coarsest = in->coarsestLvl;
   for (int l = 0; l < c->cfg.levels; l++) {
     if (!c->haveK[l]) return set_error(DMV_ERR_STATE, "dmv_ct_set_K(level) first");
     T.n[l] = c->n[l]; T.w[l] = c->w[l]; T.h[l] = c->h[l];
@@ -1105,50 +929,43 @@ int dmv_ct_track(dmv_ct* c, const dmv_ct_track_args* in, dmv_ct_track_result* ou
     const float Kl[9] = {c->fx[l], 0.f, c->cx[l], 0.f, c->fy[l], c->cy[l], 0.f, 0.f, 1.f};
     inv3_cofactor(Kl, T.Ki[l]);
     T.u[l] = c->d_u[l]; T.v[l] = c->d_v[l]; T.id[l] = c->d_id[l]; T.col[l] = c->d_col[l]; T.img[l] = c->d_img[l];
-    if (l <= in->coarsestLvl) maxn = std::max(maxn, c->n[l]);
   }
-  T.G = (maxn + CT_THREADS - 1) / CT_THREADS;
-  int dev_sms = 0;
-  CK(cudaDeviceGetAttribute(&dev_sms, cudaDevAttrMultiProcessorCount, c->device));
   for (int i = 0; i < 9; i++) T.R0[i] = in->R[i];
   for (int i = 0; i < 3; i++) T.t0[i] = in->t[i];
   T.a0 = in->a; T.b0 = in->b; T.ref_a = in->ref_a; T.ref_b = in->ref_b;
   T.ref_exposure = in->ref_exposure; T.new_exposure = in->new_exposure;
   T.huber = c->huber; T.cutoffTH = in->coarseCutoffTH; T.affModeA = in->affineOptModeA; T.affModeB = in->affineOptModeB;
   for (int i = 0; i < 5; i++) T.minRes[i] = in->minResForAbort[i];
-  T.partial = c->d_partial; T.bar = c->d_bar; T.out = c->h_out;
+  T.out = c->h_out;
   if (c->cluster_size == 0) {  // probe once: the largest cluster the device schedules for this kernel (16 needs the non-portable opt-in)
     c->cluster_size = -1;
-    const char* env = getenv("DMV_CT_GRID");   // A/B switch: DMV_CT_GRID=1 keeps the chip-wide cooperative-grid version
-    if (!(env && atoi(env) != 0) && ct_make_tensor_maps(c) == DMV_OK) {
-      CK(cudaFuncSetAttribute(ct_track_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CTCSmem)));
-      cudaFuncSetAttribute(ct_track_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    const int rc = ct_make_tensor_maps(c);
+    if (rc != DMV_OK) return rc;
+    c->cluster_size = -2;
+    CK(cudaFuncSetAttribute(ct_track_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CTCSmem)));
+    cudaFuncSetAttribute(ct_track_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    cudaGetLastError();
+    for (int nc : {16, 8, 4}) {
+      cudaLaunchConfig_t cfg = {};
+      cfg.gridDim = dim3(nc); cfg.blockDim = dim3(CTC_THREADS); cfg.dynamicSmemBytes = sizeof(CTCSmem); cfg.stream = c->stream;
+      cudaLaunchAttribute at[1];
+      at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = nc; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+      cfg.attrs = at; cfg.numAttrs = 1;
+      int ncl = 0;
+      if (cudaOccupancyMaxActiveClusters(&ncl, ct_track_cluster_kernel, &cfg) == cudaSuccess && ncl >= 1) { c->cluster_size = nc; break; }
       cudaGetLastError();
-      for (int nc : {16, 8, 4}) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(nc); cfg.blockDim = dim3(CTC_THREADS); cfg.dynamicSmemBytes = sizeof(CTCSmem); cfg.stream = c->stream;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = nc; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        int ncl = 0;
-        if (cudaOccupancyMaxActiveClusters(&ncl, ct_track_cluster_kernel, &cfg) == cudaSuccess && ncl >= 1) { c->cluster_size = nc; break; }
-        cudaGetLastError();
-      }
     }
   }
-  if (c->cluster_size > 0) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(c->cluster_size); cfg.blockDim = dim3(CTC_THREADS); cfg.dynamicSmemBytes = sizeof(CTCSmem); cfg.stream = c->stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = c->cluster_size; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    CK(cudaLaunchKernelEx(&cfg, ct_track_cluster_kernel, T, *c->maps));
-  } else {
-    if (T.G > dev_sms) return set_error(DMV_ERR_INVALID, "%d reference points need %d co-resident CTAs, the device has %d SMs: use dmv_ct_calc_res_gs", maxn, T.G, dev_sms);
-    CK(cudaMemsetAsync(c->d_bar, 0, sizeof(unsigned int), c->stream));
-    void* args[] = {&T};
-    CK(cudaLaunchCooperativeKernel((void*)ct_track_kernel, dim3(T.G), dim3(CT_THREADS), args, 0, c->stream));  // co-residency of all CTAs guaranteed
-  }
+  if (c->cluster_size == -1) return set_error(DMV_ERR_CUDA, "dmv_ct_track: the TMA descriptors of the level planes could not be encoded");
+  if (c->cluster_size < 0)
+    return set_error(DMV_ERR_CUDA, "dmv_ct_track: no cluster of 16, 8 or 4 CTAs (%d threads, %zu B shared memory each) fits on device %d", CTC_THREADS,
+                     sizeof(CTCSmem), c->device);
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(c->cluster_size); cfg.blockDim = dim3(CTC_THREADS); cfg.dynamicSmemBytes = sizeof(CTCSmem); cfg.stream = c->stream;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = c->cluster_size; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+  cfg.attrs = at; cfg.numAttrs = 1;
+  CK(cudaLaunchKernelEx(&cfg, ct_track_cluster_kernel, T, *c->maps));
   c->launches++;
   CK(cudaStreamSynchronize(c->stream));
   c->staging_busy = false;
@@ -1159,13 +976,29 @@ int dmv_ct_track(dmv_ct* c, const dmv_ct_track_args* in, dmv_ct_track_result* ou
   for (int i = 0; i < 5; i++) out->lastResiduals[i] = o[14 + i];
   for (int i = 0; i < 3; i++) out->flowIndicators[i] = o[19 + i];
   out->trackingGood = (int)o[22]; out->iterations = (int)o[23]; out->evaluations = (int)o[24]; out->status = (int)o[25];
-  if (out->status == 1) return set_error(DMV_ERR_CUDA, "ct_track_kernel: grid barrier timed out");
   return DMV_OK;
 }
 
 void dmv_ip_default_settings(dmv_ip_settings* s) {
   s->maxPixSearch = 0.027f; s->trace_stepsize = 1.0f; s->trace_GNThreshold = 0.1f; s->trace_extraSlackOnTH = 1.2f; s->trace_slackInterval = 1.5f;
   s->trace_minImprovementFactor = 2.f; s->huberTH = 9.f; s->trace_GNIterations = 3; s->minTraceTestRadius = 2;
+}
+
+// the immature-point staging buffers d_ip / h_ip, shared by dmv_ct_make_coarse_depth, dmv_ct_init_points and dmv_ct_trace_points_multi:
+// grown to hold n points of CT_IP_WORDS words each (23 read-only floats, 7 in/out words and the set index of dmv_ct_trace_points_multi)
+// plus the per-frame tables (14 floats for each of up to 64 host frames)
+constexpr int CT_IP_WORDS = 31;
+static int ct_reserve_ip(dmv_ct* c, int n) {
+  if (n <= c->ip_cap) return DMV_OK;
+  cudaFree(c->d_ip);
+  cudaFreeHost(c->h_ip);
+  c->d_ip = nullptr; c->h_ip = nullptr; c->ip_cap = 0;
+  const int cap = std::max(n, 2048);
+  const size_t bytes = sizeof(float) * ((size_t)CT_IP_WORDS * cap + 14 * 64);
+  CK(cudaMalloc(&c->d_ip, bytes));
+  CK(cudaMallocHost(&c->h_ip, bytes));
+  c->ip_cap = cap;
+  return DMV_OK;
 }
 
 // CoarseTracker::setCoarseTrackingRef -> makeCoarseDepthL0 (CoarseTracker.cpp:L138-295) on the device (ct_depth.cu); the reference frame is
@@ -1186,12 +1019,9 @@ int dmv_ct_make_coarse_depth(dmv_ct* c, int n, const float* Ku, const float* Kv,
     CK(cudaMallocHost(&c->cd_totals, sizeof(int) * DMV_MAX_PYR_LEVELS));
   }
   // ---- the splat's only order-dependent part on the host: points hitting the same pixel are folded in input order (L144-160)
-  if (n > c->ip_cap) {
-    if (c->d_ip) cudaFree(c->d_ip);
-    if (c->h_ip) cudaFreeHost(c->h_ip);
-    c->ip_cap = std::max(n, 2048);
-    CK(cudaMalloc(&c->d_ip, sizeof(float) * ((size_t)31 * c->ip_cap + 14 * 64)));
-    CK(cudaMallocHost(&c->h_ip, sizeof(float) * ((size_t)31 * c->ip_cap + 14 * 64)));
+  {
+    const int rc = ct_reserve_ip(c, n);
+    if (rc != DMV_OK) return rc;
   }
   if (c->staging_busy) { CK(cudaStreamSynchronize(c->stream)); c->staging_busy = false; }
   const size_t cap = c->ip_cap;
@@ -1254,12 +1084,9 @@ int dmv_ct_init_points(dmv_ct* c, int n, const int32_t* u, const int32_t* v, flo
   for (int i = 0; i < n; i++)
     if (u[i] < 2 || v[i] < 2 || u[i] >= c->w[0] - 3 || v[i] >= c->h[0] - 3) return set_error(DMV_ERR_INVALID, "point %d (%d,%d): the pattern leaves the image", i, u[i], v[i]);
   CK(cudaSetDevice(c->device));
-  if (n > c->ip_cap) {
-    if (c->d_ip) cudaFree(c->d_ip);
-    if (c->h_ip) cudaFreeHost(c->h_ip);
-    c->ip_cap = std::max(n, 2048);
-    CK(cudaMalloc(&c->d_ip, sizeof(float) * ((size_t)31 * c->ip_cap + 14 * 64)));
-    CK(cudaMallocHost(&c->h_ip, sizeof(float) * ((size_t)31 * c->ip_cap + 14 * 64)));
+  {
+    const int rc = ct_reserve_ip(c, n);
+    if (rc != DMV_OK) return rc;
   }
   if (c->staging_busy) { CK(cudaStreamSynchronize(c->stream)); c->staging_busy = false; }
   const size_t cap = c->ip_cap;
@@ -1298,13 +1125,9 @@ int dmv_ct_trace_points_multi(dmv_ct* c, int nsets, const dmv_ip_points* sets, c
   }
   if (n == 0) return DMV_OK;
   CK(cudaSetDevice(c->device));
-  const int words = 31;   // 23 read-only floats, 7 in/out words and the set index per point
-  if (n > c->ip_cap) {
-    if (c->d_ip) cudaFree(c->d_ip);
-    if (c->h_ip) cudaFreeHost(c->h_ip);
-    c->ip_cap = std::max(n, 2048);
-    CK(cudaMalloc(&c->d_ip, sizeof(float) * ((size_t)words * c->ip_cap + 14 * 64)));
-    CK(cudaMallocHost(&c->h_ip, sizeof(float) * ((size_t)words * c->ip_cap + 14 * 64)));
+  {
+    const int rc = ct_reserve_ip(c, n);
+    if (rc != DMV_OK) return rc;
   }
   if (nsets > 64) return set_error(DMV_ERR_INVALID, "at most 64 host frames per call");
   if (c->staging_busy) { CK(cudaStreamSynchronize(c->stream)); c->staging_busy = false; }
@@ -1328,7 +1151,7 @@ int dmv_ct_trace_points_multi(dmv_ct* c, int nsets, const dmv_ip_points* sets, c
     at += m;
   }
   std::memcpy(hb + o_tab, tables14, sizeof(float) * 14 * (size_t)nsets);
-  CK(cudaMemcpyAsync(c->d_ip, hb, sizeof(float) * ((size_t)words * cap + 14 * (size_t)nsets), cudaMemcpyHostToDevice, c->stream));
+  CK(cudaMemcpyAsync(c->d_ip, hb, sizeof(float) * ((size_t)CT_IP_WORDS * cap + 14 * (size_t)nsets), cudaMemcpyHostToDevice, c->stream));
   IPTraceArgs A;
   std::memset(&A, 0, sizeof(A));
   A.n = n; A.w = c->w[0]; A.h = c->h[0];

@@ -300,7 +300,7 @@ int dmv_ct_calc_res_gs(dmv_ct* ct, int level, const float RKi[9], const float t[
  * doubling, level repeat) runs on the device; the host gets the tracked pose back.  Same semantics as driving dmv_ct_calc_res_gs from the
  * host loop: R,t = lastToNew_out (refToNew, row-major), a,b = aff_g2l_out; on an aborted track (NaN residual or > 1.5*minResForAbort)
  * trackingGood = 0, status = 2 and R,t,a,b are returned unchanged, like the reference's early `return false`.
- * Needs all ceil(n/256) CTAs co-resident (n <= 148*256 reference points per level); otherwise DMV_ERR_INVALID. */
+ * Runs on one thread-block cluster and takes any reference-point count up to max_points per level. */
 typedef struct dmv_ct_track_args {
   double R[9], t[3];          /* in: initial refToNew */
   double a, b;                /* in: initial aff_g2l of the new frame */

@@ -67,6 +67,22 @@ def test_calc_res_gs_parity(capi, orc, synth, levels):
     g.close()
 
 
+def test_track_abort_returns_input_pose(capi, orc, synth):
+    """dmv_ct_track aborted at its first level (minResForAbort = 0): status 2, not good, and R, t, a, b exactly as passed in, like the
+    reference's early `return false`; lastResiduals of the aborted level as the oracle's, the levels never reached stay NaN."""
+    T, oct_, g = _setup(capi, orc, synth, 0)
+    R0, t0, a0, b0 = np.eye(3), np.zeros(3), 0.0, 0.0
+    r_o = oct_.track(R0, t0, a0, b0, coarsest=3, minRes=np.zeros(5))
+    r_g = g.track(R0, t0, a0, b0, coarsest=3, minRes=np.zeros(5))
+    assert r_g["status"] == 2 and r_g["good"] == 0
+    np.testing.assert_array_equal(r_g["R"], R0)
+    np.testing.assert_array_equal(r_g["t"], t0)
+    assert r_g["a"] == a0 and r_g["b"] == b0
+    np.testing.assert_allclose(r_g["lastResiduals"][3], r_o["lastResiduals"][3], rtol=2e-3)
+    assert np.isnan(r_g["lastResiduals"][[0, 1, 2, 4]]).all()
+    g.close()
+
+
 def test_device_pyramid_matches_host(capi, orc, synth):
     """dmv_ct_upload_new_image (FrameHessian::makeImages on the device) gives the same calcRes/GS as uploading host pyramids."""
     T, oct_, g = _setup(capi, orc, synth, 0)

@@ -66,8 +66,11 @@ def test_device_pyramid_frames(hostapi, orc, synth):
 
 @pytest.mark.parametrize("device_lm", [False, True], ids=["host_lm", "device_lm"])
 @pytest.mark.parametrize("levels", [4, 5])
-def test_track_newest_coarse(hostapi, orc, synth, levels, device_lm):
-    T = synth.make_tracking_pair(seed=4321, levels=levels if levels == 5 else 0)
+@pytest.mark.parametrize("npts", [2000, 12000])
+def test_track_newest_coarse(hostapi, orc, synth, npts, levels, device_lm):
+    """npts=12000 puts 54 195 reference points on level 0: more than a 16-CTA cluster keeps in registers (16 384), so dmv_ct_track
+    streams the rest of the level from global memory."""
+    T = synth.make_tracking_pair(seed=4321, levels=levels if levels == 5 else 0, npts=npts)
     oct_ = orc.CoarseTracker(T["w"], T["h"], T["K"], levels if levels == 5 else 0)
     oct_.make_coarse_depth(T["Ku"], T["Kv"], T["new_idepth"], T["HdiF"], T["pyr_ref"])
     oct_.set_new_frame(T["pyr_new"])
