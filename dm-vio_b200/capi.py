@@ -135,6 +135,19 @@ class CIEvalResult(C.Structure):
                 ("alphaOpt", C.c_float), ("n_good_new", C.c_int)]
 
 
+class PSSettings(C.Structure):
+    _fields_ = [("minGradHistCut", C.c_float), ("minGradHistAdd", C.c_float), ("gradDownweightPerLevel", C.c_float), ("selectDirectionDistribution", C.c_int)]
+
+
+class PSArgs(C.Structure):
+    _fields_ = [("density", C.c_float), ("recursionsLeft", C.c_int), ("thFactor", C.c_float), ("currentPotential", C.c_int), ("B256", C.c_void_p),
+                ("settings", C.POINTER(PSSettings))]
+
+
+class PSResult(C.Structure):
+    _fields_ = [("numHaveSub", C.c_int), ("currentPotential", C.c_int)]
+
+
 # every symbol declared in include/dmvio_b200.h (checked by tests/test_capi_symbols.py)
 SYMBOLS = [
     "dmv_last_error", "dmv_version", "dmv_device_count",
@@ -147,6 +160,7 @@ SYMBOLS = [
     "dmv_ct_create", "dmv_ct_destroy", "dmv_ct_set_K", "dmv_ct_set_ref", "dmv_ct_make_coarse_depth", "dmv_ct_get_ref", "dmv_ct_upload_new", "dmv_ct_upload_new_image", "dmv_ct_set_huber",
     "dmv_ci_create", "dmv_ci_destroy", "dmv_ci_set_K", "dmv_ci_upload_first", "dmv_ci_upload_new", "dmv_ci_set_points", "dmv_ci_calc_res_and_gs", "dmv_ci_kernel_launch_count",
     "dmv_ct_calc_res_gs", "dmv_ct_track", "dmv_ip_default_settings", "dmv_ct_init_points", "dmv_ct_trace_points", "dmv_ct_trace_points_multi", "dmv_ct_set_timing", "dmv_ct_last_timing", "dmv_ct_kernel_launch_count", "dmv_ct_last_point_evaluations",
+    "dmv_ps_default_settings", "dmv_ct_select_pixels", "dmv_ct_make_new_traces",
 ]
 
 
@@ -214,6 +228,10 @@ def lib():
         L.dmv_ct_calc_res_gs.argtypes = [vp, C.c_int, f32p, f32p, f32p, C.c_float, C.c_float, C.c_int, f64p, f64p, f64p, C.POINTER(C.c_int)]
         L.dmv_ct_track.argtypes = [vp, C.POINTER(CTTrackArgs), C.POINTER(CTTrackResult)]
         L.dmv_ct_init_points.argtypes = [vp, C.c_int, i32p, i32p, f32p, f32p, f32p, f32p, i32p]
+        L.dmv_ps_default_settings.argtypes = [C.POINTER(PSSettings)]
+        L.dmv_ps_default_settings.restype = None
+        L.dmv_ct_select_pixels.argtypes = [vp, C.POINTER(PSArgs), vp, C.POINTER(PSResult)]
+        L.dmv_ct_make_new_traces.argtypes = [vp, C.POINTER(PSArgs), C.c_int, C.POINTER(C.c_int), vp, vp, vp, vp, vp, vp, vp, C.POINTER(PSResult)]
         L.dmv_ct_trace_points.argtypes = [vp, C.POINTER(IPPoints), f32p, f32p, f32p, vp]
         L.dmv_ct_trace_points_multi.argtypes = [vp, C.c_int, vp, f32p, vp]
         L.dmv_ct_set_timing.argtypes = [vp, C.c_int]
@@ -477,6 +495,7 @@ class CT:
         self.h = vp()
         check(self.L.dmv_ct_create(C.byref(cfg), C.byref(self.h)))
         self.levels = levels
+        self._wh = (w, h)
 
     def close(self):
         if self.h:
@@ -538,6 +557,44 @@ class CT:
         a = [np.zeros(n.value, np.float32) for _ in range(4)]
         check(self.L.dmv_ct_get_ref(self.h, lvl, C.byref(n), *[x.ctypes.data for x in a]))
         return dict(u=a[0], v=a[1], idepth=a[2], color=a[3])
+
+    @staticmethod
+    def _ps_args(density, recursionsLeft, thFactor, potential, B, settings):
+        keep = []
+        a = PSArgs(float(density), int(recursionsLeft), float(thFactor), int(potential), None, None)
+        if B is not None:
+            Bc = _c(B, np.float32)
+            assert Bc.size == 256
+            keep.append(Bc)
+            a.B256 = Bc.ctypes.data
+        if settings is not None:
+            st = PSSettings(float(settings[0]), float(settings[1]), float(settings[2]), int(settings[3]))
+            keep.append(st)
+            a.settings = C.pointer(st)
+        return a, keep
+
+    def select_pixels(self, density, recursionsLeft=1, thFactor=1.0, potential=3, B=None, settings=None, want_map=True):
+        """PixelSelector::makeMaps on the resident frame -> (map as uint8 h x w or None, numHaveSub, potential after the call).
+        B = CalibHessian::B (256 floats) or None; settings = (minGradHistCut, minGradHistAdd, gradDownweightPerLevel, selectDirectionDistribution)."""
+        a, keep = self._ps_args(density, recursionsLeft, thFactor, potential, B, settings)
+        r = PSResult()
+        w, h = self._wh
+        m = np.zeros((h, w), np.float32) if want_map else None
+        check(self.L.dmv_ct_select_pixels(self.h, C.byref(a), None if m is None else m.ctypes.data, C.byref(r)))
+        return (None if m is None else m.astype(np.uint8)), r.numHaveSub, r.currentPotential
+
+    def make_new_traces(self, density, recursionsLeft=1, thFactor=1.0, potential=3, B=None, settings=None, cap=None):
+        """FullSystem::makeNewTraces on the resident frame -> (dict u, v, type, color, weights, gradH, energyTH; numHaveSub; potential after)"""
+        a, keep = self._ps_args(density, recursionsLeft, thFactor, potential, B, settings)
+        w, h = self._wh
+        cap = w * h if cap is None else cap
+        P = dict(u=np.zeros(cap, np.int32), v=np.zeros(cap, np.int32), type=np.zeros(cap, np.float32), color=np.zeros((cap, 8), np.float32),
+                 weights=np.zeros((cap, 8), np.float32), gradH=np.zeros((cap, 4), np.float32), energyTH=np.zeros(cap, np.float32))
+        n = C.c_int(0)
+        r = PSResult()
+        check(self.L.dmv_ct_make_new_traces(self.h, C.byref(a), cap, C.byref(n), *[P[k].ctypes.data for k in ("u", "v", "type", "color", "weights",
+                                                                                                               "gradH", "energyTH")], C.byref(r)))
+        return {k: x[:n.value] for k, x in P.items()}, r.numHaveSub, r.currentPotential
 
     def init_points(self, u, v):
         """ImmaturePoint constructor on the resident frame; same dict layout as oracle.orc.ip_init."""

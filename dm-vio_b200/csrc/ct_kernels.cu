@@ -12,6 +12,8 @@
 #include "inv3.h"
 #include "ip_trace.h"
 #include "ct_depth.h"
+#include "ps_select.h"
+#include <cmath>
 #include <cuda.h>
 #include <unordered_map>
 #include <algorithm>
@@ -702,6 +704,8 @@ struct dmv_ct {
   CTMaps* maps = nullptr;      // TMA descriptors of the level planes (host copy; passed as a kernel parameter)
   long long launches = 0;
   float last_ms[4] = {0, 0, 0, 0};
+  unsigned resident = 0;       // bit l: a frame's level l is resident (dmv_ct_upload_new_image sets every level, dmv_ct_upload_new its own)
+  PSState* ps = nullptr;       // pixel selection buffers (ps_select.cu), allocated on first use
 };
 
 #define CK(call)                                                                                   \
@@ -778,6 +782,7 @@ int dmv_ct_destroy(dmv_ct* c) {
   if (c->ev[1]) cudaEventDestroy(c->ev[1]);
   if (c->stream) cudaStreamDestroy(c->stream);
   delete c->maps;
+  if (c->ps) { ps_free(*c->ps); delete c->ps; }
   delete c;
   return DMV_OK;
 }
@@ -823,6 +828,7 @@ int dmv_ct_upload_new(dmv_ct* c, int l, const float* dIp) {
   c->launches++;
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(c->stream));
+  c->resident |= 1u << l;
   return DMV_OK;
 }
 
@@ -847,6 +853,7 @@ int dmv_ct_upload_new_image(dmv_ct* c, const float* image) {
   // no synchronisation: every consumer (dmv_ct_calc_res_gs / dmv_ct_track) runs on the same stream and synchronises itself; the image
   // was copied into the handle's pinned staging buffer above, so the caller's buffer is already free
   c->staging_busy = true;
+  c->resident = (1u << c->cfg.levels) - 1;
   return DMV_OK;
 }
 
@@ -1184,6 +1191,91 @@ int dmv_ct_trace_points(dmv_ct* c, const dmv_ip_points* p, const float KRKi[9], 
   float tab[14];
   std::memcpy(tab, KRKi, 36); std::memcpy(tab + 9, Kt, 12); std::memcpy(tab + 12, aff, 8);
   return dmv_ct_trace_points_multi(c, 1, p, tab, settings);
+}
+
+// PixelSelector::makeMaps on the resident frame (ps_select.cu): argument checks shared by dmv_ct_select_pixels / dmv_ct_make_new_traces
+static int ct_select(dmv_ct* c, const dmv_ps_args* a, dmv_ps_result* r) {
+  if (!c || !a || !r) return set_error(DMV_ERR_INVALID, "null argument");
+  if (c->w[0] % 16 || c->h[0] % 16) return set_error(DMV_ERR_INVALID, "pixel selection needs w and h divisible by 16 (have %dx%d)", c->w[0], c->h[0]);
+  if (c->cfg.levels < 3) return set_error(DMV_ERR_INVALID, "pixel selection reads pyramid levels 0..2 (handle has %d)", c->cfg.levels);
+  if (!(a->density > 0.f) || !std::isfinite(a->density) || a->currentPotential < 1 || !std::isfinite(a->thFactor))
+    return set_error(DMV_ERR_INVALID, "bad dmv_ps_args (density %g, currentPotential %d, thFactor %g)", a->density, a->currentPotential, a->thFactor);
+  if ((c->resident & 7u) != 7u) return set_error(DMV_ERR_STATE, "no frame resident: upload one first (dmv_ct_upload_new_image, or dmv_ct_upload_new of levels 0..2)");
+  CK(cudaSetDevice(c->device));
+  if (!c->ps) c->ps = new PSState();
+  int rc = ps_alloc(*c->ps, c->w[0], c->h[0]);
+  if (rc != DMV_OK) return rc;
+  const float4* img[3] = {c->d_img[0], c->d_img[1], c->d_img[2]};
+  return ps_make_maps(*c->ps, img, *a, c->stream, &c->launches, r);
+}
+
+int dmv_ct_select_pixels(dmv_ct* c, const dmv_ps_args* a, float* map_out, dmv_ps_result* r) {
+  dmv_ps_result res;
+  const int rc = ct_select(c, a, &res);
+  if (rc != DMV_OK) return rc;
+  if (map_out) {
+    CK(cudaMemcpyAsync(map_out, c->ps->map, sizeof(float) * c->w[0] * c->h[0], cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+  }
+  *r = res;
+  return DMV_OK;
+}
+
+// FullSystem::makeNewTraces (FullSystem.cpp:L1640-1665): selection, compaction in raster order and the ImmaturePoint constructor
+// (ip_trace.cu) on the device; one download of the points, of which the host keeps those with a finite energyTH
+int dmv_ct_make_new_traces(dmv_ct* c, const dmv_ps_args* a, int cap, int* n, int32_t* u, int32_t* v, float* type, float* color8, float* weights8,
+                           float* gradH4, float* energyTH, dmv_ps_result* r) {
+  if (!n || cap < 0 || (cap > 0 && (!u || !v || !type || !color8 || !weights8 || !gradH4 || !energyTH))) return set_error(DMV_ERR_INVALID, "null argument");
+  dmv_ps_result res;
+  int rc = ct_select(c, a, &res);
+  if (rc != DMV_OK) return rc;
+  rc = ct_reserve_ip(c, std::max(res.numHaveSub, 1));
+  if (rc != DMV_OK) return rc;
+  // the compaction writes u | v | type at words 28, 29, 30 x cap (cap >= numHaveSub >= the count m); the constructor then works in the
+  // stride-m layout u | v | color*8 | weights*8 | gradH*4 | energyTH | ok | type, which ends before word 25 x cap
+  const size_t cap_ip = c->ip_cap;
+  float* d = c->d_ip;
+  float* scratch = d + 28 * cap_ip;
+  int m = 0;
+  rc = ps_compact(*c->ps, 2 /* patternPadding */, reinterpret_cast<int*>(scratch), reinterpret_cast<int*>(scratch + cap_ip), scratch + 2 * cap_ip, c->stream,
+                  &c->launches, &m);
+  if (rc != DMV_OK) return rc;
+  int kept = 0;
+  if (m > 0) {
+    const size_t M = (size_t)m;
+    float* hb = c->h_ip;
+    CK(cudaMemcpyAsync(d, scratch, sizeof(float) * M, cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaMemcpyAsync(d + M, scratch + cap_ip, sizeof(float) * M, cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaMemcpyAsync(d + 24 * M, scratch + 2 * cap_ip, sizeof(float) * M, cudaMemcpyDeviceToDevice, c->stream));
+    IPInitArgs A;
+    A.n = m; A.w = c->w[0];
+    A.outlierTHSumComponent = 50.f * 50.f; A.outlierTH = 12.f * 12.f; A.overallEnergyTHWeight = 1.f;  // util/settings.cpp:L111-114, L159
+    A.u = reinterpret_cast<const int*>(d); A.v = reinterpret_cast<const int*>(d + M);
+    A.color = d + 2 * M; A.weights = d + 10 * M; A.gradH = d + 18 * M; A.energyTH = d + 22 * M; A.ok = reinterpret_cast<int*>(d + 23 * M);
+    A.img = c->d_img[0];
+    launch_ip_init(A, c->stream);
+    c->launches++;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(hb, d, sizeof(float) * 25 * M, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    const int* ok = reinterpret_cast<const int*>(hb + 23 * M);
+    for (int i = 0; i < m; i++) kept += ok[i] != 0;
+    if (kept <= cap) {
+      const int* hu = reinterpret_cast<const int*>(hb);
+      const int* hv = reinterpret_cast<const int*>(hb + M);
+      for (int i = 0, k = 0; i < m; i++) {
+        if (!ok[i]) continue;
+        u[k] = hu[i]; v[k] = hv[i]; type[k] = hb[24 * M + i];
+        std::memcpy(color8 + 8 * k, hb + 2 * M + 8 * i, 32); std::memcpy(weights8 + 8 * k, hb + 10 * M + 8 * i, 32);
+        std::memcpy(gradH4 + 4 * k, hb + 18 * M + 4 * i, 16); energyTH[k] = hb[22 * M + i];
+        k++;
+      }
+    }
+  }
+  *n = kept;
+  if (kept > cap) return set_error(DMV_ERR_INVALID, "%d new immature points, cap %d", kept, cap);
+  *r = res;
+  return DMV_OK;
 }
 
 // library-internal: the resident level-0 float4 plane of the coarse-tracker handle (dmv_ba_adopt_frame copies it device-to-device)

@@ -349,7 +349,7 @@ typedef struct dmv_ip_points {
   float *lastTraceUV2, *lastTracePixelInterval;
 } dmv_ip_points;
 /* ImmaturePoint::ImmaturePoint (ImmaturePoint.cpp:L34-63) for n integer pixels (u, v) of the frame resident in the handle (the frame that
- * just became a keyframe, FullSystem::makeNewTraces, FullSystem.cpp:L1284-1330): pattern colours, weights (setting_outlierTHSumComponent = 50*50),
+ * just became a keyframe, FullSystem::makeNewTraces, FullSystem.cpp:L1640-1665): pattern colours, weights (setting_outlierTHSumComponent = 50*50),
  * gradH (row-major 2x2), energyTH (= 8 * setting_outlierTH * setting_overallEnergyTHWeight^2 = 1152); ok[i] = 0 where a colour is not finite
  * (energyTH = NaN, the caller drops the point like the reference).  Bit-identical to the CPU code. */
 int dmv_ct_init_points(dmv_ct* ct, int n, const int32_t* u, const int32_t* v, float* color8, float* weights8, float* gradH4, float* energyTH, int32_t* ok);
@@ -359,6 +359,39 @@ int dmv_ct_trace_points(dmv_ct* ct, const dmv_ip_points* pts, const float KRKi[9
 /* The same for the immature points of SEVERAL host keyframes at once (the whole loop of FullSystem::traceNewCoarse, FullSystem.cpp:L554-575):
  * sets[k] = the points hosted by keyframe k, tables14 = per host [KRKi 9 | Kt 3 | aff 2]; one upload, one launch, one download. */
 int dmv_ct_trace_points_multi(dmv_ct* ct, int nsets, const dmv_ip_points* sets, const float* tables14, const dmv_ip_settings* settings);
+
+/* ------------------------------------------------------------------------------------------------
+ * Pixel selection for new keyframes  ==  PixelSelector::makeMaps (FullSystem/PixelSelector2.cpp:L94-454) and FullSystem::makeNewTraces
+ * (FullSystem.cpp:L1640-1665) on the frame resident in the coarse-tracker handle: the frame last given to dmv_ct_upload_new_image, or to
+ * dmv_ct_upload_new for levels 0, 1 and 2 (the same contract as dmv_ct_init_points).  absSquaredGrad of levels 0..2 is computed from the
+ * resident {I, dx, dy} planes.  Results are BIT-IDENTICAL to the reference's CPU code and identical from call to call.
+ * The selector's state (PixelSelector::currentPotential) travels through the call: the caller owns it, as FullSystem owns pixelSelector.
+ * DMV_ERR_INVALID: w or h not divisible by 16, fewer than 3 levels, density <= 0, currentPotential < 1; DMV_ERR_STATE: no frame resident.
+ * ------------------------------------------------------------------------------------------------ */
+typedef struct dmv_ps_settings {       /* util/settings.cpp:L167-170 */
+  float minGradHistCut;                /* 0.5 */
+  float minGradHistAdd;                /* 7 */
+  float gradDownweightPerLevel;        /* 0.75 */
+  int selectDirectionDistribution;     /* 1 */
+} dmv_ps_settings;
+void dmv_ps_default_settings(dmv_ps_settings* s);
+typedef struct dmv_ps_args {
+  float density;          /* numWant: setting_desiredImmatureDensity (makeNewTraces) or densities[0]*w*h (CoarseInitializer::setFirst) */
+  int recursionsLeft;     /* 1 */
+  float thFactor;         /* 1 (makeNewTraces), 2 (setFirst) */
+  int currentPotential;   /* PixelSelector::currentPotential before the call (3 for a new selector) */
+  const float* B256;      /* CalibHessian::B for the gamma weighting of absSquaredGrad; NULL = HCalib == 0 / setting_gammaWeightsPixelSelect == 0 */
+  const dmv_ps_settings* settings;     /* NULL = defaults */
+} dmv_ps_args;
+typedef struct dmv_ps_result { int numHaveSub; int currentPotential; } dmv_ps_result;  /* makeMaps' return value; the potential after the call */
+/* PixelSelector::makeMaps(fh, map_out, density, recursionsLeft, false, thFactor).  map_out: w*h floats of 0/1/2/4 (may be NULL). */
+int dmv_ct_select_pixels(dmv_ct* ct, const dmv_ps_args* a, float* map_out, dmv_ps_result* r);
+/* FullSystem::makeNewTraces: makeMaps, then an ImmaturePoint (as dmv_ct_init_points) for every selected pixel with x, y in
+ * [patternPadding+1, dim-patternPadding-2), in raster order; points whose energyTH is not finite are dropped, as the reference does.
+ * Out: *n points of u, v, type (the map value), color8, weights8, gradH4 (row-major 2x2), energyTH.  If more than cap points are kept, only
+ * *n (the count needed) is written and DMV_ERR_INVALID is returned. */
+int dmv_ct_make_new_traces(dmv_ct* ct, const dmv_ps_args* a, int cap, int* n, int32_t* u, int32_t* v, float* type,
+                           float* color8, float* weights8, float* gradH4, float* energyTH, dmv_ps_result* r);
 
 /* enable/disable the CUDA-event timing of dmv_ct_calc_res_gs (off by default); dmv_ct_last_timing()[0] = kernel milliseconds */
 int dmv_ct_set_timing(dmv_ct* ct, int enable);
